@@ -260,6 +260,28 @@ def test_bench_cpu_extras_functions():
     assert v["vae_encode_s"] > 0 and v["vae_decode_s"] > 0
 
 
+def test_bench_dump_outputs_float32_and_seeded_sample_past_the_limit(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: each array lands as <name>.npy in float32, exactly; past the size limit every run writes
+    the same sample of elements, within the limit."""
+    import importlib.util
+    from pathlib import Path
+
+    spec = importlib.util.spec_from_file_location("bench_mod", Path(__file__).resolve().parent.parent / "bench.py")
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    img = np.arange(2 * 4 * 4 * 3, dtype=np.uint8).reshape(2, 4, 4, 3)
+    b.dump_outputs(tmp_path / "a", {"images": img})
+    got = np.load(tmp_path / "a" / "images.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, img)
+    monkeypatch.setattr(b, "DUMP_LIMIT_BYTES", 256)
+    big = np.random.default_rng(1).random((20, 20))
+    for d in ("b", "c"):
+        b.dump_outputs(tmp_path / d, {"x": big, "y": big[:5]})
+    x1, x2, y1 = (np.load(tmp_path / d / n) for d, n in (("b", "x.npy"), ("c", "x.npy"), ("b", "y.npy")))
+    assert x1.dtype == np.float32 and x1.nbytes + y1.nbytes <= 256 and len(x1) > len(y1) > 0
+    assert np.array_equal(x1, x2) and np.isin(x1, big.astype(np.float32)).all()
+
+
 def test_ctypes_signatures_match_the_header():
     """every function include/b2f.h declares is bound in _lib._SIGNATURES with the same number and kinds of arguments
     (pointer / int / int64 / float / double / size_t) — a mismatch corrupts the call silently."""
