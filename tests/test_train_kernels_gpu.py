@@ -26,22 +26,30 @@ def _randn(*shape, g, scale=1.0):
 
 
 # ------------------------------------------------------------------ GEMM dgrad / wgrad
-@pytest.mark.parametrize("B,M,N,K", [
-    (1, 128, 128, 64),        # one tile, one k-block
-    (1, 200, 136, 72),        # ragged everything
-    (2, 300, 256, 512),       # batched rows, 1-CTA 128-wide kernel
-    (1, 2336, 3072, 3072),    # to_out dgrad at 512^2 (pair kernel)
-    (1, 2336, 3072, 9216),    # QKV dgrad (pair kernel, long K)
-    (2, 1024, 1024, 4096),    # pair kernel with batch
-    (1, 4736, 512, 256),      # 1-CTA 256-wide kernel
-])
+# ((B, M, N, K), the kernel gemm_dgrad picks on a 148-SM B200); test_kernel_dispatch_gpu.py checks the labels
+DGRAD_CASES = [
+    ((1, 128, 128, 64), "gemm1cta128"),        # one tile, one k-block
+    ((1, 200, 136, 72), "gemm1cta128"),        # ragged everything
+    ((2, 300, 256, 512), "gemm1cta128"),       # batched rows
+    ((1, 2336, 3072, 3072), "gemm2cta256"),    # to_out dgrad at 512^2
+    ((1, 2336, 3072, 9216), "gemm2cta256"),    # QKV dgrad, long K
+    ((2, 1024, 1024, 4096), "gemm1cta128"),    # batched rows: 32 pair tiles, below the pair kernel's 74
+    ((1, 4736, 512, 256), "gemm1cta128"),      # 38 pair tiles; the 256-wide 1-CTA kernel is unreachable
+    ((2, 1024, 3072, 3072), "gemm2cta256"),    # pair kernel with batch
+]
+
+
+@pytest.mark.parametrize("B,M,N,K", [shape for shape, _ in DGRAD_CASES])
 def test_gemm_dgrad(B, M, N, K):
     from gpt_image_edit_b200 import train_ops as T
+    from test_kernel_dispatch_gpu import _require_variant, _run_on_variant
 
+    variant = (dict(DGRAD_CASES)[(B, M, N, K)], 1)
+    _require_variant("dgrad", B, M, N, K, T.EPI_STORE, variant)
     g = _g(1)
     dy = _randn(B, M, K, g=g)
     w = _randn(K, N, g=g, scale=0.05)          # nn.Linear weight [out = K, in = N]
-    dx = T.linear_dgrad(dy, w)
+    dx = _run_on_variant(lambda: T.linear_dgrad(dy, w), variant)
     ref = dy.float() @ w.float()
     assert dx.shape == (B, M, N)
     assert _rel(dx, ref) < 4e-3
@@ -70,21 +78,29 @@ def test_gemm_dgrad_pitched_views_and_epilogues():
     assert _rel(out, acc.float() + base) < 4e-3
 
 
-@pytest.mark.parametrize("B,rows,M,N", [
-    (1, 64, 128, 128),
-    (1, 100, 136, 200),       # ragged: token tail inside a 64-row box, M/N tails
-    (3, 150, 256, 384),       # contraction over three batch items with a ragged tail each
-    (1, 2336, 3072, 3072),    # to_out wgrad at 512^2 (pair kernel)
-    (2, 1000, 1024, 4608),    # pair kernel, batch 2
-    (1, 288, 12288, 3584),    # MLP2 first linear
-])
+# ((B, rows, M, N), the kernel gemm_wgrad picks on a 148-SM B200)
+WGRAD_CASES = [
+    ((1, 64, 128, 128), "gemm1cta128"),
+    ((1, 100, 136, 200), "gemm1cta128"),       # ragged: token tail inside a 64-row box, M/N tails
+    ((3, 150, 256, 384), "gemm1cta128"),       # contraction over three batch items with a ragged tail each
+    ((1, 2336, 3072, 3072), "gemm2cta256"),    # to_out wgrad at 512^2
+    ((2, 1000, 1024, 4608), "gemm1cta128"),    # batch 2: 72 pair tiles, below the pair kernel's 74
+    ((1, 288, 12288, 3584), "gemm2cta256"),    # MLP2 first linear
+    ((2, 1000, 2048, 3072), "gemm2cta256"),    # pair kernel, contraction over two batch items
+]
+
+
+@pytest.mark.parametrize("B,rows,M,N", [shape for shape, _ in WGRAD_CASES])
 def test_gemm_wgrad(B, rows, M, N):
     from gpt_image_edit_b200 import train_ops as T
+    from test_kernel_dispatch_gpu import EPI_F32, _require_variant, _run_on_variant
 
+    variant = (dict(WGRAD_CASES)[(B, rows, M, N)], 2)
+    _require_variant("wgrad", B, M, N, rows, EPI_F32, variant)
     g = _g(3)
     dy = _randn(B, rows, M, g=g)
     x = _randn(B, rows, N, g=g)
-    dw = T.linear_wgrad(dy, x)
+    dw = _run_on_variant(lambda: T.linear_wgrad(dy, x), variant)
     ref = torch.einsum("brm,brn->mn", dy.float(), x.float())
     assert dw.dtype == torch.float32 and dw.shape == (M, N)
     assert _rel(dw, ref) < 1e-3
